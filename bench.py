@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Mfeatures/s (extract + match) of the B200 feature hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config {2,3,4}] [--frames F] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config {2,3,4}] [--frames F] [--impl reference] [--dump-outputs DIR]
 
 --config 2 (default, the configuration BASELINE.json's metric is quoted on): a stream of 3-fisheye 754x480 multi-camera frames,
     8-level pyramid (scale 1.2), 2000 features per camera, mdBRIEF-256 with masks; every (frame, camera) is brute-force matched
@@ -21,6 +21,11 @@ pinned HOST buffers, H2D and D2H inside the timed region.  `roofline` is the fus
 bytes per launch / CUDA-event time / measured HBM peak.  `cpu_baseline` / --impl reference: the reference's own extractor and
 matcher (oracle/_ref/libmcs_ref.so, compiled from /root/reference where that exists) on the host cores over a bounded sample,
 else the oracle port.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step returned to its caller as DIR/<name>.npy
+(float32 / float64): every image's feature and match counts, and the keypoints, descriptors, descriptor masks and matches of a
+fixed seeded sample of DUMP_IMAGES images.  The inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import json
@@ -38,6 +43,7 @@ sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "oracle"))
 
 NLEVELS = 8
+DUMP_IMAGES = 32            # images of the last step whose features --dump-outputs writes (config 2: about 21 MB)
 CONFIGS = {
     2: dict(n_cams=3, w=754, h=480, nfeatures=2000, frames=128, sharding="stream",
             workload="lafida-3cam-754x480-stream, 8 levels x1.2, 2000 feat/cam, mdBRIEF-256+masks, greedy brute-force match vs previous frame"),
@@ -317,6 +323,28 @@ def host_views(cfg, cam, mask, scene, F):
     return out
 
 
+def dump_outputs(path, out, nmatches, matches12):
+    """--dump-outputs: out = the packed feature views of the last timed step; nmatches [B] and matches12 (config 2 and 4: [B, cap]
+    per image, config 3: one index per keypoint of the frame view) as the step's matcher returned them.  Rows past an image's
+    feature count are not outputs (the buffer keeps whatever an earlier step left there) and are written as zeros / -1."""
+    from multicol_slam_b200.ctypes_defs import KEYPOINT_DTYPE
+    d = pathlib.Path(path)
+    d.mkdir(parents=True, exist_ok=True)
+    counts = out["counts"].cpu().numpy()
+    B, cap = out["kps"].shape[:2]
+    pick = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_IMAGES), replace=False))
+    valid = (np.arange(cap)[None, :] < counts[pick, None])[..., None]
+    kps = out["kps"].cpu().numpy()[pick].view(KEYPOINT_DTYPE)[..., 0]
+    arrays = {"counts": counts, "nmatches": np.asarray(nmatches).reshape(-1), "sample_images": pick,
+              "keypoints": np.where(valid, np.stack([kps[f].astype(np.float64) for f in KEYPOINT_DTYPE.names], -1), 0.0),
+              "descriptors": np.where(valid, out["desc"].cpu().numpy()[pick], 0).astype(np.float32),
+              "descriptor_masks": np.where(valid, out["dmask"].cpu().numpy()[pick], 0).astype(np.float32)}
+    m12 = np.asarray(matches12)
+    arrays["matches12"] = np.where(valid[..., 0], m12.reshape(B, cap)[pick], -1) if m12.size == B * cap else m12
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", np.asarray(a, np.float32 if a.dtype == np.float32 else np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------------------------------
 # GPU arm
 # ---------------------------------------------------------------------------------------------------------------------------
@@ -330,6 +358,7 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--ref-frames", type=int, default=8, help="frames per step of the CPU reference arm (config 2)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     cfg_id, cfg = args.config, CONFIGS[args.config]
     if args.impl == "reference":
@@ -394,6 +423,7 @@ def main():
     m12b, nmatb = torch.empty_like(m12), torch.empty_like(nmat)
     sf = np.array([float(np.float32(1.2)) ** l for l in range(NLEVELS)])
     stats = {"matches": 0}
+    last = {}               # matcher outputs of configs 3 / 4 in the last step (--dump-outputs)
 
     # matching targets of configs 3 / 4, built from the features of a first extraction
     scene = None
@@ -436,8 +466,9 @@ def main():
         t_c = time.perf_counter()
         mp = api.MapPoints(np.zeros(len(scene["world"]), np.uint8), iv, lv, px, py, vc, scene["mp_desc"], scene["mp_dmask"])
         mt = api.cORBmatcher(0.8, False, ds, True)
-        n, _ = mt.SearchByProjection(Fr, mp, 3.0)
+        n, last["matches12"] = mt.SearchByProjection(Fr, mp, 3.0)
         t_d = time.perf_counter()
+        last["nmatches"] = [n]
         stats["matches"] = n
         stats["match_call_ms"] = (t_d - t_m3) * 1e3
         stats["parts_ms"] = {"wait_extract+d2h": (t_a - t_m3) * 1e3, "frame_view": (t_b - t_a) * 1e3, "mcs_project_mappoints": (t_c - t_b) * 1e3,
@@ -449,8 +480,9 @@ def main():
         valid1 = (np.arange(cap)[None, :] < counts[:, None]).astype(np.uint8).reshape(-1)
         # every key frame of the batch against the database as its own SearchByBoW(KF1, KF2): independent "already matched" state
         # per frame, the K-best lists of all frames from one launch
-        nms, _ = api.match_bruteforce_batch_device(v["desc"].view(B * cap, ds), v["dmask"].view(B * cap, ds), valid1, np.arange(B + 1) * cap,
+        nms, last["matches12"] = api.match_bruteforce_batch_device(v["desc"].view(B * cap, ds), v["dmask"].view(B * cap, ds), valid1, np.arange(B + 1) * cap,
                                                    scene["db_t"], scene["dbm_t"], None, m.TH_LOW_, 0.9, stream=stream)
+        last["nmatches"] = nms
         stats["matches"] = int(nms.sum())
         stats["match_call_ms"] = (time.perf_counter() - t_m) * 1e3      # includes waiting for this step's extraction (the counts read)
 
@@ -531,6 +563,11 @@ def main():
         barrier()
         ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:          # before the e2e and roofline passes below reuse the buffers
+        if cfg_id == 2:
+            dump_outputs(args.dump_outputs, out, nmat.cpu().numpy(), m12.cpu().numpy())
+        else:
+            dump_outputs(args.dump_outputs, out, last["nmatches"], last["matches12"])
     feats_rank = int(out["counts"].sum().item())
     redo_n = int(redo.sum().item()) if cfg_id == 2 else 0
     matches_rank = int(nmat.sum().item()) if cfg_id == 2 else stats["matches"]

@@ -1,6 +1,6 @@
 """GPU parity against outputs of the REFERENCE'S OWN extractor: the CUDA path (through the C ABI) vs the fixtures
 tests/golden/ref_extract_*.npz, which tests/golden/make_ref_extract_golden.py wrote from oracle/_ref/libmcs_ref.so
-(/root/reference/src/mdBRIEFextractorOct.cpp, cam_model_omni.cpp, misc.cpp compiled in place).  Bit-exact: keypoint
+(the original project's src/mdBRIEFextractorOct.cpp, cam_model_omni.cpp, misc.cpp compiled in place).  Bit-exact: keypoint
 bytes (incl. the IC angle float), descriptor and mask bytes, pyramid and mask-pyramid levels.  Covers the configuration the
 reference ships (plain ORB, 400 features), its init extractor, BASELINE.json configs 1-4 and parameter corners."""
 import glob
@@ -10,6 +10,8 @@ import zlib
 
 import numpy as np
 import pytest
+
+from ref_golden import RECORD, RefGolden, not_recording
 
 pytestmark = pytest.mark.gpu
 GOLD = pathlib.Path(__file__).resolve().parent / "golden"
@@ -22,6 +24,7 @@ def crc(a):
     return zlib.crc32(np.ascontiguousarray(a).tobytes())
 
 
+@not_recording
 @pytest.mark.parametrize("path", FIXTURES, ids=lambda p: pathlib.Path(p).stem[12:])
 def test_gpu_equals_reference_fixture(api, path):
     from multicol_slam_b200 import synth
@@ -49,14 +52,19 @@ def test_gpu_equals_reference_fixture(api, path):
 
 
 def test_gpu_equals_reference_live(api, cams):
-    """where oracle/_ref travelled to this box: the reference library itself, on fresh seeds, next to the CUDA path"""
+    """the reference extractor on three more seeds and modes (tests/golden/ref_pin_gpu.npz, tests/ref_golden.py) next to the CUDA path"""
     import ref_mcs_api as ra
-    if not ra.available():
-        pytest.skip("oracle/_ref/libmcs_ref.so not present")
     from multicol_slam_b200 import synth
+    gold = RefGolden("ref_pin_gpu")
+    cases = []
     for seed, (mode, nf) in enumerate([(dict(), 400), (dict(do_dbrief=True), 900), (dict(do_dbrief=True, learn_masks=True), 2000)]):
         cam = cams[seed]
         img, mask = synth.frame(cam, 900 + seed), synth.mirror_mask(cam)
-        rk, rd, rm = ra.RefExtractor(nfeatures=nf, **mode).extract(img, mask, cam)
+        ref = gold(f"extract/{seed}", lambda: tuple(crc(a) for a in ra.RefExtractor(nfeatures=nf, **mode).extract(img, mask, cam)))
+        cases.append((mode, nf, cam, img, mask, ref))
+    gold.save()
+    if RECORD:
+        pytest.skip("reference outputs recorded")
+    for mode, nf, cam, img, mask, ref in cases:
         k, d, m = api.mdBRIEFextractorOct(nfeatures=nf, do_dBrief=mode.get("do_dbrief", False), learnMasks=mode.get("learn_masks", False))(img, mask, cam)
-        assert k.tobytes() == rk.tobytes() and np.array_equal(d, rd) and np.array_equal(m, rm)
+        assert (crc(k), crc(d), crc(m)) == ref
