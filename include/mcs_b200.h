@@ -477,6 +477,49 @@ int  mcs_search_by_bow(const uint8_t* desc1, const uint8_t* mask1, const uint8_t
                        const int32_t* fv2_nodes, const int32_t* fv2_offsets, int32_t n_fv2, const int32_t* fv2_features,
                        int32_t dim, int32_t th_low, double nnratio, int32_t* match_of_2, int32_t* nmatches);
 
+/* ---- key-frame database: loop and relocalisation candidates (ref src/cMultiKeyFrameDatabase.cpp) ------------------------ */
+/* cMultiKeyFrameDatabase(voc) (ref :36-40).  The inverted file, the BowVectors given to add() and the per-key-frame query
+ * fields live on the device that is current at creation; every call checks that it still is (MCS_ERR_INVALID otherwise).
+ * The entry points are serialised by one internal mutex (the reference shares the database between the tracking and the
+ * loop-closing threads).  KL scoring (type 3): MCS_ERR_UNSUPPORTED (a device log() need not round like the host's; the other
+ * five types use + - * / sqrt |.| only and reproduce mcs_bow_score bit for bit).
+ * Key-frame ids are cMultiKeyFrame::mnId: non-negative, below 2^30 here (MCS_ERR_UNSUPPORTED beyond: the per-key-frame fields
+ * mnLoopQuery / mnLoopWords / mLoopScore / mnRelocQuery / mnRelocWords / mRelocScore are arrays indexed by id).  Those fields
+ * start at 0 (0.0 for the scores; the reference leaves all but the two query ids uninitialised, src/cMultiKeyFrame.cpp:44-45),
+ * outlive erase() and clear() and carry from one query to the next, as on the reference's key frames.
+ * A BowVector is (words ascending, strictly, each < voc size; values), as mcs_bow_vectors returns it; MCS_ERR_INVALID otherwise. */
+typedef struct mcs_keyframe_db mcs_keyframe_db;
+int  mcs_kfdb_create(const mcs_vocabulary* voc, mcs_keyframe_db** out);
+void mcs_kfdb_destroy(mcs_keyframe_db* db);
+/* add(pKF) (ref :43-50): appends kf_id to the list of every word of its BowVector, after the entries already there; a second add
+ * of the same id appends it again (it then counts twice).  The BowVector is kept as pKF->mBowVec for scoring and erase. */
+int  mcs_kfdb_add(mcs_keyframe_db* db, int64_t kf_id, const int32_t* bow_words, const double* bow_values, int32_t n_bow);
+/* erase(pKF) (ref :52-73): removes the first (oldest) entry of kf_id from the list of every word of its latest BowVector.
+ * An id that was never added: MCS_OK, nothing changes. */
+int  mcs_kfdb_erase(mcs_keyframe_db* db, int64_t kf_id);
+/* clear() (ref :75-79): empties every list; the per-key-frame fields and stored BowVectors stay. */
+int  mcs_kfdb_clear(mcs_keyframe_db* db);
+/* DetectLoopCandidates(pKF, minScore) (ref :82-215; call site src/cLoopClosing.cpp:155) and DetectRelocalisationCandidates(F)
+ * (ref :217-327; call site src/cTracking.cpp:1134).
+ * kf_id / frame_id: pKF->mnId / F->mnId (non-negative); bow: pKF->mBowVec / F->mBowVec.
+ * connected[n_connected]: pKF->GetConnectedKeyFrames() (never listed; their mnLoopWords are still reset and counted, ref :102-111).
+ * covis: row id = GetBestCovisibilityKeyFrames(10) of key frame id as the reference reads it at query time, covis[id*10 + j],
+ * -1 = none, rows for ids 0..n_covis_rows-1 (missing rows: no neighbours).  Entries must be -1 or an id.
+ * candidates: key-frame ids in the reference's order (first encounter: query words ascending, each list in add order; pBestKF
+ * deduplicated keeping the first).  MCS_ERR_CAPACITY with *n_candidates = the required count when `capacity` is too small;
+ * the query has run all the same (its effect on the per-key-frame fields stays, as in the reference), so a retry is a new
+ * query.  A capacity of 1 + the largest id added or named in covis always suffices.
+ * Relocalisation reads a neighbour's mRelocScore whenever mnRelocQuery == F->mnId (ref :293), also when this query did not
+ * score it: the value is then the one of the last query that did (0.0 if none). */
+int  mcs_kfdb_detect_loop_candidates(mcs_keyframe_db* db, int64_t kf_id, const int32_t* bow_words, const double* bow_values,
+                                     int32_t n_bow, const int64_t* connected, int32_t n_connected, const int64_t* covis,
+                                     int64_t n_covis_rows, double min_score, int64_t* candidates, int32_t capacity,
+                                     int32_t* n_candidates);
+int  mcs_kfdb_detect_relocalisation_candidates(mcs_keyframe_db* db, int64_t frame_id, const int32_t* bow_words,
+                                               const double* bow_values, int32_t n_bow, const int64_t* covis,
+                                               int64_t n_covis_rows, int64_t* candidates, int32_t capacity,
+                                               int32_t* n_candidates);
+
 /* ---- multi-GPU: one camera (or stream chunk) per GPU, ONE allgather of the packed feature buffer (SURVEY 8e) -------------- */
 /* Packed feature buffer of a batch of n_images images: the four output arrays of the batched extractor in one allocation,
  *   [ counts int32[n_images] | mcs_keypoint[n_images][capacity] | desc u8[n_images][capacity][dim] | dmask u8[n_images][capacity][dim] ]

@@ -5,6 +5,8 @@ operator/matcher interface for this path:
         (ref include/mdBRIEFextractorOct.h:333-368, src/mdBRIEFextractorOct.cpp:1244-1337)
     cORBmatcher(nnratio, checkOri, featDim, havingMasks).SearchByProjection / SearchForInitialization /
         SearchByBoW(KF1, KF2)   (ref include/cORBmatcher.h:58-158, src/cORBmatcher.cpp:46-166, 579-726, 885-966)
+    ORBVocabulary(voc).transform / score and KeyFrameDatabase(voc).add / erase / clear / DetectLoopCandidates /
+        DetectRelocalisationCandidates   (ref include/cMultiKeyFrameDatabase.h, src/cMultiKeyFrameDatabase.cpp)
 
 There is no CPU fallback: the shared library must be present (build it with `python __graft_entry__.py`)
 and every compute call needs an sm_100 device, otherwise it raises.
@@ -1141,3 +1143,65 @@ class ORBVocabulary:
         s = C.c_double(0)
         _check(lib().mcs_bow_score(self._h, _p(w1), _p(x1), len(w1), _p(w2), _p(x2), len(w2), C.byref(s)))
         return s.value
+
+
+class KeyFrameDatabase:
+    """Mirror of cMultiKeyFrameDatabase (ref include/cMultiKeyFrameDatabase.h, src/cMultiKeyFrameDatabase.cpp): the inverted
+    file over `voc`'s words and the per-key-frame query fields live on the GPU (mcs_kfdb_*).  Key frames are named by their
+    mnId; bow = (words, values) as ORBVocabulary.transform returns them; covis = int64 [n, 10], row id = the ten best
+    covisibility key frames of key frame id at query time (-1 = none).  The Detect* calls return int64 arrays of key-frame ids
+    in the reference's order."""
+
+    def __init__(self, voc: ORBVocabulary):
+        self._voc = voc                      # the database reads the vocabulary's size and scoring type; keep it alive
+        self._top = 0
+        self._h = C.c_void_p()
+        _check(lib().mcs_kfdb_create(voc._h, C.byref(self._h)))
+
+    def __del__(self):
+        if getattr(self, "_h", None):
+            lib().mcs_kfdb_destroy(self._h)
+            self._h = None
+
+    @staticmethod
+    def _bow(bow):
+        return np.ascontiguousarray(bow[0], np.int32), np.ascontiguousarray(bow[1], np.float64)
+
+    def add(self, kf_id, bow):
+        w, v = self._bow(bow)
+        if len(w) != len(v):
+            raise ValueError("BowVector words and values differ in length")
+        _check(lib().mcs_kfdb_add(self._h, C.c_int64(kf_id), _p(w), _p(v), len(w)))
+        self._top = max(self._top, int(kf_id) + 1)
+
+    def erase(self, kf_id):
+        _check(lib().mcs_kfdb_erase(self._h, C.c_int64(kf_id)))
+
+    def clear(self):
+        _check(lib().mcs_kfdb_clear(self._h))
+
+    def _args(self, bow, covis):
+        w, v = self._bow(bow)
+        if len(w) != len(v):
+            raise ValueError("BowVector words and values differ in length")
+        cv = np.ascontiguousarray(np.zeros((0, 10), np.int64) if covis is None else covis, np.int64)
+        if cv.ndim != 2 or cv.shape[1] != 10:
+            raise ValueError("covis must be an int64 array [n, 10]")
+        # every candidate is an added key frame or a neighbour named in covis, so this capacity always suffices
+        out = np.zeros(max(self._top, int(cv.max()) + 1 if cv.size else 0, 1), np.int64)
+        return w, v, cv, out
+
+    def DetectLoopCandidates(self, kf_id, bow, connected, covis, minScore):
+        w, v, cv, out = self._args(bow, covis)
+        conn = np.ascontiguousarray(np.zeros(0) if connected is None else connected, np.int64)
+        n = C.c_int32(0)
+        _check(lib().mcs_kfdb_detect_loop_candidates(self._h, C.c_int64(kf_id), _p(w), _p(v), len(w), _p(conn), len(conn), _p(cv),
+                                                     C.c_int64(len(cv)), C.c_double(minScore), _p(out), len(out), C.byref(n)))
+        return out[:n.value].copy()
+
+    def DetectRelocalisationCandidates(self, frame_id, bow, covis):
+        w, v, cv, out = self._args(bow, covis)
+        n = C.c_int32(0)
+        _check(lib().mcs_kfdb_detect_relocalisation_candidates(self._h, C.c_int64(frame_id), _p(w), _p(v), len(w), _p(cv),
+                                                               C.c_int64(len(cv)), _p(out), len(out), C.byref(n)))
+        return out[:n.value].copy()

@@ -13,6 +13,7 @@
 #include "../../include/mcs_b200.h"
 #include "kernels.h"
 #include "dev_scratch.h"
+#include "vocabulary.h"
 
 using namespace mcs;
 
@@ -35,11 +36,6 @@ int bfail(int code, const std::string& msg) { mcs_set_error_(msg); return code; 
 
 }  // namespace
 
-struct mcs_vocabulary {
-    int k = 0, L = 0, scoring = 0, weighting = 0, n_nodes = 0, n_words = 0, device = 0;
-    Dev child_off, child_ids, desc, word_of_node, weight;
-    VocabularyDev view{};
-};
 
 extern "C" {
 
